@@ -8,6 +8,7 @@ own CPU implementation timed on this box's host cores.
 
   python bench.py --gpus 1 --steps 20 --warmup 3          # our arm
   python bench.py --impl reference --steps 2 --warmup 1   # the unmodified reference (CPU)
+  python bench.py --dump-outputs DIR ...                  # also save a sample of the result (float32 .npy)
   torchrun ... bench.py --gpus N ...                      # one rank per GPU, weak scaling:
                                                           # each rank owns one 512^3 Z slab
 
@@ -360,6 +361,21 @@ def slab_parity_check(dev, rank, world, passes, peer_halo_factory):
   return bool(flag.item())
 
 
+DUMP_VOXELS = 1 << 23            # 32 MiB of float32 over all ranks
+
+
+def dump_outputs(path, out, rank, world):
+  """Write a fixed, seeded sample of this rank's edtsq result (the distances a caller of the timed
+  path receives) as float32 to path/edtsq.npy (path/edtsq_rank<r>.npy with several ranks), so that
+  two builds run with the same arguments can be compared output for output."""
+  import torch
+  idx = np.random.default_rng(12345 + rank).integers(0, out.numel(), DUMP_VOXELS // world)
+  idx.sort()
+  sample = out.reshape(-1)[torch.from_numpy(idx).to(out.device)].cpu().numpy().astype(np.float32)
+  os.makedirs(path, exist_ok=True)
+  np.save(os.path.join(path, "edtsq.npy" if world == 1 else "edtsq_rank%d.npy" % rank), sample)
+
+
 def ours(args):
   import torch
   import torch.distributed as dist
@@ -455,6 +471,8 @@ def ours(args):
   stop.record(stream)
   barrier()
   elapsed_ms = start.elapsed_time(stop)
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, result["out"] if world > 1 else f_dev, rank, world)
   if True:
     # per-pass device times: the same K steps once more with the library recording CUDA events
     # around every pass (on the launch stream, no syncs).  Kept out of the timed region above
@@ -727,7 +745,13 @@ def main():
   ap.add_argument("--warmup", type=int, default=3)
   ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
   ap.add_argument("--no-cpu-baseline", action="store_true")
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="after the timed steps, write a seeded sample of the last step's edtsq result to DIR/*.npy")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl == "reference":
+    ap.error("--dump-outputs is only available for --impl ours")
   if args.impl == "reference":
     reference_arm(args)
   else:

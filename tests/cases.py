@@ -8,6 +8,8 @@ checked against them with exact equality, as the reference does (`np.all(result 
 random_volume()/RANDOM_SPECS drive the randomized differential tests (CUDA vs oracle) and the
 committed fixtures under tests/golden/ (compiled reference -> oracle, see make_golden.py).
 """
+import hashlib
+
 import numpy as np
 
 I = np.inf
@@ -200,3 +202,26 @@ def random_graph_case(seed):
   an = ANISOTROPIES[(seed // 5) % len(ANISOTROPIES)][:nd]
   kwargs = dict(anisotropy=an, black_border=bool((seed // 2) % 2))
   return labels, graph, kwargs
+
+
+# cases whose reference outputs are stored as digests (tests/golden/reference_digests.json)
+DIGEST_SEEDS = range(300)                 # random_case: edtsq of each, edt and sdf of every third
+DIGEST_GRAPH_SEEDS = range(100, 160)      # random_graph_case: edtsq and sdf
+
+
+def cfg2_volume():
+  """BASELINE.json configs[1]: 512^3 uint32 iid labels 0..255, Fortran order."""
+  rng = np.random.default_rng(0)
+  return np.asfortranarray(rng.integers(0, 256, (512, 512, 512), dtype=np.uint32))
+
+
+def digest(a):
+  """SHA-256 of an array's dtype, shape and values in C order, with -0.0 folded onto +0.0 and one
+  NaN for every NaN, so that two float arrays of one dtype have the same digest exactly when
+  np.array_equal(a, b, equal_nan=True) holds for them."""
+  a = np.asarray(a)
+  if a.dtype.kind == "f":
+    a = np.where(np.isnan(a), a.dtype.type(np.nan), a + a.dtype.type(0))
+  h = hashlib.sha256(("%s %s " % (a.dtype.str, a.shape)).encode())
+  h.update(np.ascontiguousarray(a).tobytes())
+  return h.hexdigest()

@@ -3,10 +3,11 @@
 The oracle (oracle/edt_oracle.c) is only trusted because it reproduces
   (a) the reference's own golden vectors (tests/cases.py, restated from automated_test.py),
   (b) the committed fixtures produced by the compiled reference (tests/golden/),
-  (c) the compiled reference itself, live, wherever oracle/_ref exists,
+  (c) digests of the compiled reference's outputs on a few hundred more seeded cases (tests/golden/),
   (d) a brute-force evaluation of the definition on tiny volumes.
 All comparisons are exact (bit-for-bit), as in the reference's tests.
 """
+import json
 import os
 
 import numpy as np
@@ -15,6 +16,7 @@ import pytest
 import cases
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_vectors.npz")
+DIGESTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")
 
 
 def same(a, b):
@@ -95,22 +97,24 @@ def test_fixture_cases_are_reproducible():
     assert labels.flags.f_contiguous == z["s%d_labels" % seed].flags.f_contiguous
 
 
-def test_live_against_compiled_reference(oracle, reference):
-  if reference is None:
-    pytest.skip("oracle/_ref not built here")
-  for seed in range(300):
+def test_live_against_compiled_reference(oracle):
+  """The oracle against the compiled reference's outputs on 300 random and 60 voxel-graph cases,
+  stored as digests (bit-exact, see cases.digest) by make_golden.py."""
+  with open(DIGESTS) as fh:
+    want = json.load(fh)
+  for seed in cases.DIGEST_SEEDS:
     labels, kwargs = cases.random_case(seed)
-    assert same(oracle.edtsq(labels, **kwargs), reference.edtsq(labels, **kwargs)), seed
+    ref = want["random_case"][str(seed)]
+    assert cases.digest(oracle.edtsq(labels, **kwargs)) == ref["edtsq"], seed
     if seed % 3 == 0:
-      assert same(oracle.sdf(labels, **kwargs), reference.sdf(labels, **kwargs)), seed
-      assert same(oracle.edt(labels, **kwargs), reference.edt(labels, **kwargs)), seed
-  for seed in range(100, 160):
+      assert cases.digest(oracle.sdf(labels, **kwargs)) == ref["sdf"], seed
+      assert cases.digest(oracle.edt(labels, **kwargs)) == ref["edt"], seed
+  for seed in cases.DIGEST_GRAPH_SEEDS:
     labels, graph, kwargs = cases.random_graph_case(seed)
+    ref = want["random_graph_case"][str(seed)]
     with np.errstate(invalid="ignore"):
-      assert same(oracle.edtsq(labels, voxel_graph=graph, **kwargs),
-                  reference.edtsq(labels, voxel_graph=graph, **kwargs)), seed
-      assert same(oracle.sdf(labels, voxel_graph=graph, **kwargs),
-                  reference.sdf(labels, voxel_graph=graph, **kwargs)), seed
+      assert cases.digest(oracle.edtsq(labels, voxel_graph=graph, **kwargs)) == ref["edtsq"], seed
+      assert cases.digest(oracle.sdf(labels, voxel_graph=graph, **kwargs)) == ref["sdf"], seed
 
 
 def test_definition_bruteforce(oracle):

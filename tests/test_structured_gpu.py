@@ -3,8 +3,8 @@
 * Long runs with varying heights (Voronoi cells, balls) at 512 rows per line -- the inputs that
   exercise the lower-envelope stages of the later-axis kernel (hull build per chunk, stitching
   across chunk boundaries, read-out) -- compared LIVE with the compiled, unmodified reference
-  (oracle/_ref) where it is present (it is on the GPU box), else with the C restatement.
-* The whole 512^3 headline volume (BASELINE configs[1]) against the compiled reference.
+  (oracle/_ref) where it is present, else with the C restatement.
+* The whole 512^3 headline volume (BASELINE configs[1]) against the compiled reference's stored result.
 * edt.each / each_cuda / label_stats_cuda against the reference's own edt.each
   (src/edt.pyx:951-994) and against plain numpy masking.
 """
@@ -71,15 +71,17 @@ def test_structured_256_cubed_live(edt, oracle, reference, kind):
               ref("edt", lab, anisotropy=(0.7, 1.3, 2.9), black_border=True), (kind, 256, "non-integer"))
 
 
-def test_cfg2_full_volume_live(edt, reference):
-  # BASELINE.json configs[1], the whole 512^3 volume against the compiled reference
-  if reference is None:
-    pytest.skip("compiled reference (oracle/_ref) not present")
+def test_cfg2_full_volume_live(edt):
+  # BASELINE.json configs[1], the whole 512^3 volume against the compiled reference's result, stored
+  # as a digest (bit-exact, see cases.digest) by tests/golden/make_golden.py
+  import json
   import os
-  rng = np.random.default_rng(0)
-  lab = np.asfortranarray(rng.integers(0, 256, (512, 512, 512), dtype=np.uint32))
-  want = reference.edtsq(lab, anisotropy=(1, 1, 1), black_border=False, parallel=os.cpu_count() or 1)
-  assert_same(edt.edtsq(lab, anisotropy=(1, 1, 1)), want, "cfg2 512^3")
+  import cases
+  with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")) as fh:
+    want = json.load(fh)["cfg2_512"]["edtsq"]
+  got = edt.edtsq(cases.cfg2_volume(), anisotropy=(1, 1, 1))
+  assert got.dtype == np.float32 and got.shape == (512, 512, 512)
+  assert cases.digest(got) == want, "cfg2 512^3 differs from the compiled reference's edtsq"
 
 
 def test_wide_lines_and_rows_that_are_not_stored(edt, oracle, reference):
