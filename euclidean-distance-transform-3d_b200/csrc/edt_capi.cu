@@ -48,22 +48,6 @@ EncodeTiledFn tensor_map_encoder() {
   return encode;
 }
 
-size_t tile_smem_bytes(int n, int tx, int rows_alloc) {
-  const int nchunks = (n + 31) >> 5;
-  return (size_t)rows_alloc * tx * 4 + (size_t)nchunks * tx * 12 + (size_t)((n + 3) & ~1) * 4 + 16 +
-         (size_t)nchunks * tx +    // + one flag byte per (chunk, line)
-         (size_t)tx * 4 + 4;       // + one word per line: chunks holding a run start
-}
-
-// Will launch_later() take the shared-memory tile kernel for this geometry?  (same conditions)
-bool tile_path_ok(const LineGeom& g, const DeviceCache& dc) {
-  if (!((int64_t)g.n * g.line_stride + 64 < (1LL << 32) && g.n <= 4096 && g.inner_count < (1LL << 31))) return false;
-  const int nb = (g.n + 255) / 256;
-  int br = (g.n + nb - 1) / nb;
-  if (nb > 1) br = (br + 3) & ~3;
-  return tile_smem_bytes(g.n, 8, br * nb) <= (size_t)dc.max_smem_optin;
-}
-
 cudaError_t scratch_alloc(DeviceCache& dc, void** p, size_t bytes, cudaStream_t stream) {
   if (dc.pool) return cudaMallocFromPoolAsync(p, bytes, dc.pool, stream);
   return cudaMallocAsync(p, bytes, stream);
@@ -380,27 +364,31 @@ int check_dims(int label_bytes, int ndim, int64_t& sx, int64_t& sy, int64_t& sz)
   return 0;
 }
 
-int dispatch_first(int label_bytes, const void* labels, float* f, int64_t nlines, int64_t sx, float w,
-                   int border, int flags, DeviceCache& dc, cudaStream_t s) {
+template <int B>
+struct LabelWidth {
+  static constexpr int Bytes = B;
+  using T = typename edtb200::LabelOf<B>::type;
+};
+
+// f(LabelWidth<label_bytes>()): the label width as a compile-time constant (check_dims has
+// accepted it: 1, 2, 4 or 8).
+template <class F>
+auto with_label_width(int label_bytes, F&& f) {
   switch (label_bytes) {
-    case 1: return launch_first<1>(labels, f, nlines, sx, w, border, flags, dc, s);
-    case 2: return launch_first<2>(labels, f, nlines, sx, w, border, flags, dc, s);
-    case 4: return launch_first<4>(labels, f, nlines, sx, w, border, flags, dc, s);
-    default: return launch_first<8>(labels, f, nlines, sx, w, border, flags, dc, s);
+    case 1: return f(LabelWidth<1>());
+    case 2: return f(LabelWidth<2>());
+    case 4: return f(LabelWidth<4>());
+    default: return f(LabelWidth<8>());
   }
 }
 
-// fmax: an upper bound of the finite samples in f when they are known to be integer-valued (the
-// product of earlier passes with integer weights^2), or -1: enables the integer hull tests.
-int dispatch_later(int label_bytes, const void* labels, float* f, const edtb200::LineGeom& g, float w,
-                   int lo, int hi, int flags, DeviceCache& dc, cudaStream_t s, bool pdl = false, double fmax = -1.0) {
-  switch (label_bytes) {
-    case 1: return launch_later<1>(labels, f, g, w, lo, hi, flags, dc, s, pdl, fmax);
-    case 2: return launch_later<2>(labels, f, g, w, lo, hi, flags, dc, s, pdl, fmax);
-    case 4: return launch_later<4>(labels, f, g, w, lo, hi, flags, dc, s, pdl, fmax);
-    default: return launch_later<8>(labels, f, g, w, lo, hi, flags, dc, s, pdl, fmax);
-  }
+// Kernel flags of the pass that ends a transform: square root, and the sign of sdf.
+int epilogue_flags(int flags) {
+  return ((flags & EDTB200_SQRT) ? edtb200::kSqrt : 0) | ((flags & EDTB200_SIGNED) ? edtb200::kNegate : 0);
 }
+
+// Kernel flag of sdf's first pass: the background (label 0) is a label like any other.
+int zero_label_flags(int flags) { return (flags & EDTB200_SIGNED) ? edtb200::kZeroLabel : 0; }
 
 // Largest finite value the passes along axes of lengths n[0..k) with weights w[0..k) can have
 // produced, if all their squared weights (the float products the kernels use) are integers and
@@ -417,15 +405,48 @@ double integer_bound(const float* w, const int64_t* n, int k) {
   return bound < 2147483000.0 ? bound : -1.0;
 }
 
+// {outer_count, outer_stride, inner_count, line_stride, n, tiles_per_outer} of the Y / Z pass
 edtb200::LineGeom geom_for_axis(int axis, int64_t sx, int64_t sy, int64_t sz) {
-  edtb200::LineGeom g;
-  if (axis == 1) {
-    g.outer_count = sz; g.outer_stride = sx * sy; g.inner_count = sx; g.line_stride = sx; g.n = (int)sy;
-  } else {
-    g.outer_count = 1; g.outer_stride = 0; g.inner_count = sx * sy; g.line_stride = sx * sy; g.n = (int)sz;
-  }
-  g.tiles_per_outer = 0;
-  return g;
+  if (axis == 1) return {sz, sx * sy, sx, sx, (int)sy, 0};
+  return {1, 0, sx * sy, sx * sy, (int)sz, 0};
+}
+
+int first_pass(int label_bytes, const void* labels, float* f, int64_t nlines, int64_t sx, float wx, int border,
+               int kflags, DeviceCache& dc, cudaStream_t s) {
+  return with_label_width(label_bytes, [&](auto lw) {
+    return launch_first<decltype(lw)::Bytes>(labels, f, nlines, sx, wx, border, kflags, dc, s);
+  });
+}
+
+// The Y (axis 1) or Z (axis 2) pass of a volume of sx x sy x sz voxels with weights w[0..2], after
+// the passes along the earlier axes.  `part` is the extent the call covers across its lines -- z
+// for Y, y for Z: sz / sy, or one device's share when the volume is split; the integer-hull bound
+// is that of the whole volume.
+int later_pass(int axis, int label_bytes, const void* labels, float* f, int64_t sx, int64_t sy, int64_t sz,
+               int64_t part, const float* w, int border_lo, int border_hi, int kflags, bool pdl, DeviceCache& dc,
+               cudaStream_t s) {
+  const int64_t n[2] = {sx, sy};
+  const edtb200::LineGeom g = axis == 1 ? geom_for_axis(1, sx, sy, part) : geom_for_axis(2, sx, part, sz);
+  return with_label_width(label_bytes, [&](auto lw) {
+    return launch_later<decltype(lw)::Bytes>(labels, f, g, w[axis], border_lo, border_hi, kflags, dc, s, pdl,
+                                             integer_bound(w, n, axis));
+  });
+}
+
+// Device buffer `p` of at least `need` bytes (`have` now), reallocated when too small.
+template <class T>
+cudaError_t grow(T*& p, size_t& have, size_t need) {
+  if (have >= need) return cudaSuccess;
+  if (p) cudaFree(p);
+  p = nullptr; have = 0;
+  const cudaError_t e = cudaMalloc(&p, need);
+  if (e == cudaSuccess) have = need;
+  return e;
+}
+
+// Creates the cached non-blocking stream `s` of a device on first use.
+cudaError_t ensure_stream(cudaStream_t& s) {
+  return s ? cudaSuccess : cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
 }
 
 // Optional per-pass timing for bench.py: with profiling on, every transform of this thread records
@@ -483,11 +504,10 @@ void nvtx_pop() { if (g_nvtx_pop) g_nvtx_pop(); }
 int run_passes(const void* labels, int label_bytes, int ndim, int64_t sx, int64_t sy, int64_t sz,
                float wx, float wy, float wz, int border, int flags, float* f,
                DeviceCache& dc, cudaStream_t stream) {
-  using namespace edtb200;
   // sqrt / sign are applied by whichever pass is the last one; background-as-label (sdf)
   // changes the first pass only -- later passes treat every run alike.
-  const int epilogue = ((flags & EDTB200_SQRT) ? kSqrt : 0) | ((flags & EDTB200_SIGNED) ? kNegate : 0);
-  const int zero_label = (flags & EDTB200_SIGNED) ? kZeroLabel : 0;
+  const int epilogue = epilogue_flags(flags);
+  const float w[3] = {wx, wy, wz};
   // The later passes are launched with programmatic stream serialization: the kernel before them
   // in the stream is our own previous pass, which never writes the labels, so their label staging
   // (before griddepcontrol.wait) may overlap its tail.  The per-axis entry points do not do this:
@@ -496,7 +516,6 @@ int run_passes(const void* labels, int label_bytes, int ndim, int64_t sx, int64_
   // re-read wide labels, was measured in round 1 and dropped: Y 0.261 -> 0.244, Z 0.280 -> 0.250 ms
   // but X 0.180 -> 0.350 ms at 512^3 uint32.)
   int rc = 0;
-  const edtb200::LineGeom gy = geom_for_axis(1, sx, sy, sz), gz = geom_for_axis(2, sx, sy, sz);
   // EDT_B200_VERBOSE=1: per-pass device times of every transform on stderr (SURVEY.md section 5).
   // The dump needs the passes to have finished, so a verbose transform synchronises its stream.
   static const bool verbose = getenv("EDT_B200_VERBOSE") != nullptr && atoi(getenv("EDT_B200_VERBOSE")) != 0;
@@ -504,23 +523,21 @@ int run_passes(const void* labels, int label_bytes, int ndim, int64_t sx, int64_
   if (verbose) g_profile = true;
   mark_pass(0, stream);
   nvtx_push("edt.x");
-  rc = dispatch_first(label_bytes, labels, f, sy * sz, sx, wx, border, zero_label | (ndim == 1 ? epilogue : 0), dc,
-                      stream);
+  rc = first_pass(label_bytes, labels, f, sy * sz, sx, wx, border,
+                  zero_label_flags(flags) | (ndim == 1 ? epilogue : 0), dc, stream);
   nvtx_pop();
   mark_pass(1, stream);
   if (!rc && ndim >= 2) {
     nvtx_push("edt.y");
-    const float ws[1] = {wx}; const int64_t ns[1] = {sx};
-    rc = dispatch_later(label_bytes, labels, f, gy, wy, border, border, ndim == 2 ? epilogue : 0, dc, stream,
-                        /*pdl=*/true, integer_bound(ws, ns, 1));
+    rc = later_pass(1, label_bytes, labels, f, sx, sy, sz, sz, w, border, border, ndim == 2 ? epilogue : 0,
+                    /*pdl=*/true, dc, stream);
     nvtx_pop();
     mark_pass(2, stream);
   }
   if (!rc && ndim >= 3) {
     nvtx_push("edt.z");
-    const float ws[2] = {wx, wy}; const int64_t ns[2] = {sx, sy};
-    rc = dispatch_later(label_bytes, labels, f, gz, wz, border, border, epilogue, dc, stream, /*pdl=*/true,
-                        integer_bound(ws, ns, 2));
+    rc = later_pass(2, label_bytes, labels, f, sx, sy, sz, sy, w, border, border, epilogue, /*pdl=*/true, dc,
+                    stream);
     nvtx_pop();
     mark_pass(3, stream);
   }
@@ -585,7 +602,7 @@ int edtb200_transform(const void* labels, int label_bytes, int ndim, int64_t sx,
     // pure host call: a private non-blocking stream.  With one side on the device and no stream
     // given, the legacy default stream (NULL) is kept: it is ordered after the work the caller
     // queued on the default / blocking streams that produced that buffer.
-    if (!dc->stream) CUDA_TRY(cudaStreamCreateWithFlags(&dc->stream, cudaStreamNonBlocking));
+    CUDA_TRY(ensure_stream(dc->stream));
     stream = dc->stream;
   }
   const size_t lab_bytes = (size_t)total * (size_t)label_bytes;
@@ -593,23 +610,13 @@ int edtb200_transform(const void* labels, int label_bytes, int ndim, int64_t sx,
   const void* d_labels = labels;
   float* d_out = out;
   if (!lab_dev) {
-    if (dc->labels_bytes < lab_bytes) {
-      if (dc->labels) cudaFree(dc->labels);
-      dc->labels = nullptr; dc->labels_bytes = 0;
-      CUDA_TRY(cudaMalloc(&dc->labels, lab_bytes));
-      dc->labels_bytes = lab_bytes;
-    }
+    CUDA_TRY(grow(dc->labels, dc->labels_bytes, lab_bytes));
     rc = upload(dc->labels, labels, lab_bytes, device, stream);
     if (rc) return rc;
     d_labels = dc->labels;
   }
   if (!out_dev) {
-    if (dc->dist_bytes < out_bytes) {
-      if (dc->dist) cudaFree(dc->dist);
-      dc->dist = nullptr; dc->dist_bytes = 0;
-      CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&dc->dist), out_bytes));
-      dc->dist_bytes = out_bytes;
-    }
+    CUDA_TRY(grow(dc->dist, dc->dist_bytes, out_bytes));
     d_out = dc->dist;
   }
   rc = run_passes(d_labels, label_bytes, ndim, sx, sy, sz, wx, wy, wz, border, flags, d_out, *dc, stream);
@@ -644,23 +651,15 @@ int edtb200_transform_batch(const void* const* labels, float* const* outs, int c
   DeviceCache& dc = *dcp;
   std::lock_guard<std::mutex> host_call(dc.host_call);
   const size_t lab_bytes = (size_t)total * (size_t)label_bytes, out_bytes = (size_t)total * sizeof(float);
-  auto grow = [](void** p, size_t* have, size_t need) -> cudaError_t {
-    if (*have >= need) return cudaSuccess;
-    if (*p) cudaFree(*p);
-    *p = nullptr; *have = 0;
-    cudaError_t e = cudaMalloc(p, need);
-    if (e == cudaSuccess) *have = need;
-    return e;
-  };
-  CUDA_TRY(grow(&dc.labels, &dc.labels_bytes, lab_bytes));
-  CUDA_TRY(grow(reinterpret_cast<void**>(&dc.dist), &dc.dist_bytes, out_bytes));
+  CUDA_TRY(grow(dc.labels, dc.labels_bytes, lab_bytes));
+  CUDA_TRY(grow(dc.dist, dc.dist_bytes, out_bytes));
   if (count > 1) {
-    CUDA_TRY(grow(&dc.labels2, &dc.labels2_bytes, lab_bytes));
-    CUDA_TRY(grow(reinterpret_cast<void**>(&dc.dist2), &dc.dist2_bytes, out_bytes));
+    CUDA_TRY(grow(dc.labels2, dc.labels2_bytes, lab_bytes));
+    CUDA_TRY(grow(dc.dist2, dc.dist2_bytes, out_bytes));
   }
-  if (!dc.stream) CUDA_TRY(cudaStreamCreateWithFlags(&dc.stream, cudaStreamNonBlocking));
-  if (!dc.stream_up) CUDA_TRY(cudaStreamCreateWithFlags(&dc.stream_up, cudaStreamNonBlocking));
-  if (!dc.stream_down) CUDA_TRY(cudaStreamCreateWithFlags(&dc.stream_down, cudaStreamNonBlocking));
+  CUDA_TRY(ensure_stream(dc.stream));
+  CUDA_TRY(ensure_stream(dc.stream_up));
+  CUDA_TRY(ensure_stream(dc.stream_down));
   for (int i = 0; i < 2; ++i) {
     if (!dc.ev_up[i]) CUDA_TRY(cudaEventCreateWithFlags(&dc.ev_up[i], cudaEventDisableTiming));
     if (!dc.ev_comp[i]) CUDA_TRY(cudaEventCreateWithFlags(&dc.ev_comp[i], cudaEventDisableTiming));
@@ -770,7 +769,7 @@ int edtb200_transform_voxel_graph(const void* labels, int label_bytes, const uns
   std::unique_lock<std::mutex> host_call(dc->host_call, std::defer_lock);
   if (!(in_dev && out_dev)) host_call.lock();          // staging buffers and the private stream
   if (!stream && !in_dev && !out_dev) {
-    if (!dc->stream) CUDA_TRY(cudaStreamCreateWithFlags(&dc->stream, cudaStreamNonBlocking));
+    CUDA_TRY(ensure_stream(dc->stream));
     stream = dc->stream;
   }
 
@@ -807,12 +806,10 @@ int edtb200_transform_voxel_graph(const void* labels, int label_bytes, const uns
   const int blocks = (int)std::min<int64_t>((total + threads - 1) / threads, (int64_t)dc->sm_count * 32);
   const int border = black_border != 0, as_float = (flags & EDTB200_LABELS_FLOAT) ? 1 : 0;
   uint8_t* cells = static_cast<uint8_t*>(d_cells);
-  switch (label_bytes) {
-    case 1: voxel_graph_expand_kernel<1><<<blocks, threads, 0, stream>>>(lab, gr, cells, sx, sy, sz, ndim, border, as_float); break;
-    case 2: voxel_graph_expand_kernel<2><<<blocks, threads, 0, stream>>>(lab, gr, cells, sx, sy, sz, ndim, border, as_float); break;
-    case 4: voxel_graph_expand_kernel<4><<<blocks, threads, 0, stream>>>(lab, gr, cells, sx, sy, sz, ndim, border, as_float); break;
-    default: voxel_graph_expand_kernel<8><<<blocks, threads, 0, stream>>>(lab, gr, cells, sx, sy, sz, ndim, border, as_float); break;
-  }
+  with_label_width(label_bytes, [&](auto lw) {
+    voxel_graph_expand_kernel<decltype(lw)::Bytes><<<blocks, threads, 0, stream>>>(lab, gr, cells, sx, sy, sz, ndim,
+                                                                                   border, as_float);
+  });
   VG_TRY(cudaGetLastError());
   // half the anisotropy (vg:102-107, 199-204); the sqrt is taken by the gather instead
   rc = run_passes(cells, 1, ndim, sx2, sy2, sz2, wx / 2, wy / 2, wz / 2, border, 0,
@@ -841,10 +838,10 @@ int edtb200_pass_first(const void* labels_dev, int label_bytes, int64_t sx, int6
   DeviceCache* dc = nullptr;
   rc = probe(device, &dc);
   if (rc) return rc;
-  const int kflags = ((flags & EDTB200_SQRT) ? edtb200::kSqrt : 0) |
-                     ((flags & EDTB200_SIGNED) ? edtb200::kZeroLabel : 0);
-  return dispatch_first(label_bytes, labels_dev, f_dev, sy * sz, sx, wx, black_border != 0, kflags, *dc,
-                        static_cast<cudaStream_t>(stream));
+  // EDTB200_SIGNED: background as a label, without the sign
+  const int kflags = epilogue_flags(flags & EDTB200_SQRT) | zero_label_flags(flags);
+  return first_pass(label_bytes, labels_dev, f_dev, sy * sz, sx, wx, black_border != 0, kflags, *dc,
+                    static_cast<cudaStream_t>(stream));
 }
 
 int edtb200_pass_later(const void* labels_dev, int label_bytes, int axis, int64_t sx, int64_t sy, int64_t sz,
@@ -859,11 +856,12 @@ int edtb200_pass_later(const void* labels_dev, int label_bytes, int axis, int64_
   DeviceCache* dc = nullptr;
   rc = probe(device, &dc);
   if (rc) return rc;
-  return dispatch_later(label_bytes, labels_dev, f_dev, geom_for_axis(axis, sx, sy, sz), w,
-                        border_lo != 0, border_hi != 0,
-                        ((flags & EDTB200_SQRT) ? edtb200::kSqrt : 0) |
-                            ((flags & EDTB200_SIGNED) ? edtb200::kNegate : 0),
-                        *dc, static_cast<cudaStream_t>(stream));
+  const edtb200::LineGeom g = geom_for_axis(axis, sx, sy, sz);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  return with_label_width(label_bytes, [&](auto lw) {      // no integer-hull bound: the caller's f is unknown
+    return launch_later<decltype(lw)::Bytes>(labels_dev, f_dev, g, w, border_lo != 0, border_hi != 0,
+                                             epilogue_flags(flags), *dc, s, /*pdl=*/false, /*fmax=*/-1.0);
+  });
 }
 
 int edtb200_slab_face_runs(const void* labels_dev, int label_bytes, int64_t sx, int64_t sy, int64_t sz,
@@ -882,13 +880,11 @@ int edtb200_slab_face_runs(const void* labels_dev, int label_bytes, int64_t sx, 
   const int64_t plane = sx * sy;
   const unsigned blocks = (unsigned)((plane + 255) / 256);
   const int zl = (flags & EDTB200_SIGNED) ? 1 : 0;
-  using namespace edtb200;
-  switch (label_bytes) {
-    case 1: face_runs_kernel<1><<<blocks, 256, 0, stream>>>(static_cast<const uint8_t*>(labels_dev), plane, (int)sz, high_face, halo, zl, m_dev, overflow_dev); break;
-    case 2: face_runs_kernel<2><<<blocks, 256, 0, stream>>>(static_cast<const uint16_t*>(labels_dev), plane, (int)sz, high_face, halo, zl, m_dev, overflow_dev); break;
-    case 4: face_runs_kernel<4><<<blocks, 256, 0, stream>>>(static_cast<const uint32_t*>(labels_dev), plane, (int)sz, high_face, halo, zl, m_dev, overflow_dev); break;
-    default: face_runs_kernel<8><<<blocks, 256, 0, stream>>>(static_cast<const uint64_t*>(labels_dev), plane, (int)sz, high_face, halo, zl, m_dev, overflow_dev); break;
-  }
+  with_label_width(label_bytes, [&](auto lw) {
+    using LW = decltype(lw);
+    edtb200::face_runs_kernel<LW::Bytes><<<blocks, 256, 0, stream>>>(
+        static_cast<const typename LW::T*>(labels_dev), plane, (int)sz, high_face, halo, zl, m_dev, overflow_dev);
+  });
   CUDA_TRY(cudaGetLastError());
   return 0;
 }
@@ -941,15 +937,14 @@ int edtb200_slab_face_fixup(const void* labels_dev, int label_bytes, int64_t sx,
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   const int64_t plane = sx * sy;
   const unsigned blocks = (unsigned)((plane + 255) / 256);
-  using namespace edtb200;
-  const int kflags = ((flags & EDTB200_SQRT) ? kSqrt : 0) | ((flags & EDTB200_SIGNED) ? (kNegate | kZeroLabel) : 0);
+  const int kflags = epilogue_flags(flags) | zero_label_flags(flags);
   const float w2 = wz * wz;
-  switch (label_bytes) {
-    case 1: face_fixup_kernel<1><<<blocks, 256, 0, stream>>>(static_cast<const uint8_t*>(labels_dev), f_dev, plane, (int)sz, high_face, halo, w2, static_cast<const uint8_t*>(nb_label_dev), nb_m_dev, nb_f_dev, kflags, inexact_dev); break;
-    case 2: face_fixup_kernel<2><<<blocks, 256, 0, stream>>>(static_cast<const uint16_t*>(labels_dev), f_dev, plane, (int)sz, high_face, halo, w2, static_cast<const uint16_t*>(nb_label_dev), nb_m_dev, nb_f_dev, kflags, inexact_dev); break;
-    case 4: face_fixup_kernel<4><<<blocks, 256, 0, stream>>>(static_cast<const uint32_t*>(labels_dev), f_dev, plane, (int)sz, high_face, halo, w2, static_cast<const uint32_t*>(nb_label_dev), nb_m_dev, nb_f_dev, kflags, inexact_dev); break;
-    default: face_fixup_kernel<8><<<blocks, 256, 0, stream>>>(static_cast<const uint64_t*>(labels_dev), f_dev, plane, (int)sz, high_face, halo, w2, static_cast<const uint64_t*>(nb_label_dev), nb_m_dev, nb_f_dev, kflags, inexact_dev); break;
-  }
+  with_label_width(label_bytes, [&](auto lw) {
+    using LW = decltype(lw);
+    edtb200::face_fixup_kernel<LW::Bytes><<<blocks, 256, 0, stream>>>(
+        static_cast<const typename LW::T*>(labels_dev), f_dev, plane, (int)sz, high_face, halo, w2,
+        static_cast<const typename LW::T*>(nb_label_dev), nb_m_dev, nb_f_dev, kflags, inexact_dev);
+  });
   CUDA_TRY(cudaGetLastError());
   return 0;
 }
@@ -1007,7 +1002,6 @@ cudaError_t copy_box(void* dst, size_t dst_row_bytes, int64_t dst_rows_per_slice
 int edtb200_transform_multi(const void* labels, int label_bytes, int ndim, int64_t sx, int64_t sy, int64_t sz,
                             float wx, float wy, float wz, int black_border, int flags, float* out,
                             const int* devices, int ndevices) {
-  using namespace edtb200;
   if (!devices || ndevices < 1) return fail(EDTB200_EINVAL, "no devices given");
   if (flags & (EDTB200_LABELS_ON_DEVICE | EDTB200_OUT_ON_DEVICE))
     return fail(EDTB200_EINVAL, "edtb200_transform_multi splits a HOST volume over the devices");
@@ -1027,8 +1021,7 @@ int edtb200_transform_multi(const void* labels, int label_bytes, int ndim, int64
                              nullptr);
 
   const int border = black_border != 0;
-  const int zero_label = (flags & EDTB200_SIGNED) ? kZeroLabel : 0;
-  const int epilogue = ((flags & EDTB200_SQRT) ? kSqrt : 0) | ((flags & EDTB200_SIGNED) ? kNegate : 0);
+  const float w[3] = {wx, wy, wz};
   std::vector<MultiPart> parts(G);
   for (int d = 0; d < G; ++d) {
     MultiPart& p = parts[d];
@@ -1054,7 +1047,7 @@ int edtb200_transform_multi(const void* labels, int label_bytes, int ndim, int64
       host_call = std::unique_lock<std::mutex>(dc->host_call);
       for (int o = 0; o < G; ++o)                                 // direct NVLink copies where possible
         if (o != d) { cudaDeviceEnablePeerAccess(parts[o].device, 0); cudaGetLastError(); }
-      if (!dc->stream) MULTI_TRY(cudaStreamCreateWithFlags(&dc->stream, cudaStreamNonBlocking));
+      MULTI_TRY(ensure_stream(dc->stream));
       me.stream = dc->stream;
       MULTI_TRY(cudaEventCreateWithFlags(&me.after_y, cudaEventDisableTiming));
       MULTI_TRY(cudaEventCreateWithFlags(&me.after_z, cudaEventDisableTiming));
@@ -1070,11 +1063,10 @@ int edtb200_transform_multi(const void* labels, int label_bytes, int ndim, int64
     if (!wrc) {
       const char* src = static_cast<const char*>(labels) + (size_t)me.z0 * sy * row_l;
       wrc = upload(me.lz, src, (size_t)sx * sy * me.zc * label_bytes, me.device, me.stream);
-      if (!wrc) wrc = dispatch_first(label_bytes, me.lz, me.fz, sy * me.zc, sx, wx, border, zero_label, *dc, me.stream);
-      const float ws[2] = {wx, wy};
-      const int64_t ns[2] = {sx, sy};
-      if (!wrc) wrc = dispatch_later(label_bytes, me.lz, me.fz, geom_for_axis(1, sx, sy, me.zc), wy, border, border, 0,
-                                     *dc, me.stream, /*pdl=*/true, integer_bound(ws, ns, 1));
+      if (!wrc) wrc = first_pass(label_bytes, me.lz, me.fz, sy * me.zc, sx, wx, border, zero_label_flags(flags), *dc,
+                                 me.stream);
+      if (!wrc) wrc = later_pass(1, label_bytes, me.lz, me.fz, sx, sy, sz, me.zc, w, border, border, 0,
+                                 /*pdl=*/true, *dc, me.stream);
       if (wrc) note(wrc);
       MULTI_TRY(cudaEventRecord(me.after_y, me.stream));
     }
@@ -1090,10 +1082,8 @@ int edtb200_transform_multi(const void* labels, int label_bytes, int ndim, int64
                            row_l, me.yc, src.zc, me.stream));
       }
       if (!wrc) {
-        const float ws[2] = {wx, wy};
-        const int64_t ns[2] = {sx, sy};
-        wrc = dispatch_later(label_bytes, me.ly, me.fy, geom_for_axis(2, sx, me.yc, sz), wz, border, border, epilogue,
-                             *dc, me.stream, /*pdl=*/false, integer_bound(ws, ns, 2));
+        wrc = later_pass(2, label_bytes, me.ly, me.fy, sx, sy, sz, me.yc, w, border, border, epilogue_flags(flags),
+                         /*pdl=*/false, *dc, me.stream);
         if (wrc) note(wrc);
       }
       MULTI_TRY(cudaEventRecord(me.after_z, me.stream));
@@ -1161,9 +1151,9 @@ int edtb200_slab_step(const void* labels_dev, int label_bytes, int64_t sx, int64
   if (rc) return rc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   const int border = black_border != 0;
-  const int zero_label = (flags & EDTB200_SIGNED) ? kZeroLabel : 0;
-  const int epilogue = ((flags & EDTB200_SQRT) ? kSqrt : 0) | ((flags & EDTB200_SIGNED) ? kNegate : 0);
-  const edtb200::LineGeom gy = geom_for_axis(1, sx, sy, sz), gz = geom_for_axis(2, sx, sy, sz);
+  const int zero_label = zero_label_flags(flags);
+  const int epilogue = epilogue_flags(flags);
+  const float w[3] = {wx, wy, wz};
 
   // EDT_B200_VERBOSE=1: device time of every phase of the step on stderr (synchronises the stream)
   static const bool verbose = getenv("EDT_B200_VERBOSE") != nullptr && atoi(getenv("EDT_B200_VERBOSE")) != 0;
@@ -1177,16 +1167,14 @@ int edtb200_slab_step(const void* labels_dev, int label_bytes, int64_t sx, int64
   mark_pass(0, stream);              // per-pass events for bench.py (edtb200_profile_passes), as in run_passes
   // X and Y passes: slab-local
   nvtx_push("edt.x");
-  rc = dispatch_first(label_bytes, labels_dev, f_dev, sy * sz, sx, wx, border, zero_label, *dc, stream);
+  rc = first_pass(label_bytes, labels_dev, f_dev, sy * sz, sx, wx, border, zero_label, *dc, stream);
   nvtx_pop();
   if (rc) return rc;
   stamp(1);
   mark_pass(1, stream);
   nvtx_push("edt.y");
-  const float ws[2] = {wx, wy};
-  const int64_t ns[2] = {sx, sy};
-  rc = dispatch_later(label_bytes, labels_dev, f_dev, gy, wy, border, border, 0, *dc, stream, /*pdl=*/!verbose,
-                      integer_bound(ws, ns, 1));
+  rc = later_pass(1, label_bytes, labels_dev, f_dev, sx, sy, sz, sz, w, border, border, 0, /*pdl=*/!verbose, *dc,
+                  stream);
   nvtx_pop();
   if (rc) return rc;
   stamp(2);
@@ -1205,16 +1193,12 @@ int edtb200_slab_step(const void* labels_dev, int label_bytes, int64_t sx, int64
     unsigned long long* flag_in_lo_peer = has_lo ? reinterpret_cast<unsigned long long*>(lo + L.flag_from_hi) : nullptr;
     unsigned long long* flag_in_hi_peer = has_hi ? reinterpret_cast<unsigned long long*>(hi + L.flag_from_lo) : nullptr;
     unsigned int* counter = reinterpret_cast<unsigned int*>(self + L.counter);
-#define EDT_STAGE(B, T)                                                                                          \
-    slab_stage_kernel<B><<<grid, 256, 0, stream>>>(static_cast<const T*>(labels_dev), f_dev, plane, (int)sz, halo, \
-                                                   has_lo, has_hi, set, L, step, flag_in_lo_peer, flag_in_hi_peer, counter)
-    switch (label_bytes) {
-      case 1: EDT_STAGE(1, uint8_t); break;
-      case 2: EDT_STAGE(2, uint16_t); break;
-      case 4: EDT_STAGE(4, uint32_t); break;
-      default: EDT_STAGE(8, uint64_t); break;
-    }
-#undef EDT_STAGE
+    with_label_width(label_bytes, [&](auto lw) {
+      using LW = decltype(lw);
+      slab_stage_kernel<LW::Bytes><<<grid, 256, 0, stream>>>(static_cast<const typename LW::T*>(labels_dev), f_dev,
+                                                             plane, (int)sz, halo, has_lo, has_hi, set, L, step,
+                                                             flag_in_lo_peer, flag_in_hi_peer, counter);
+    });
     CUDA_TRY(cudaGetLastError());
     nvtx_pop();
   }
@@ -1223,8 +1207,8 @@ int edtb200_slab_step(const void* labels_dev, int label_bytes, int64_t sx, int64
   mark_pass(2, stream);              // "second pass" = Y plus the face staging kernel
   // Z pass on the slab, interior faces open
   nvtx_push("edt.z");
-  rc = dispatch_later(label_bytes, labels_dev, f_dev, gz, wz, border && !has_lo, border && !has_hi, epilogue, *dc,
-                      stream, /*pdl=*/!verbose && (has_lo || has_hi), integer_bound(ws, ns, 2));
+  rc = later_pass(2, label_bytes, labels_dev, f_dev, sx, sy, sz, sy, w, border && !has_lo, border && !has_hi,
+                  epilogue, /*pdl=*/!verbose && (has_lo || has_hi), *dc, stream);
   nvtx_pop();
   if (rc) return rc;
 
@@ -1238,24 +1222,17 @@ int edtb200_slab_step(const void* labels_dev, int label_bytes, int64_t sx, int64
     const unsigned char* set_hi = has_hi ? hi + (size_t)parity * L.set_bytes : nullptr;
     const unsigned long long* flag_from_lo = reinterpret_cast<const unsigned long long*>(self + L.flag_from_lo);
     const unsigned long long* flag_from_hi = reinterpret_cast<const unsigned long long*>(self + L.flag_from_hi);
-    cudaLaunchConfig_t fcfg = {};
-    fcfg.gridDim = grid; fcfg.blockDim = dim3(256); fcfg.dynamicSmemBytes = 0; fcfg.stream = stream;
-    cudaLaunchAttribute fattr[1];
-    fattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    fattr[0].val.programmaticStreamSerializationAllowed = 1;
-    fcfg.attrs = fattr;
-    fcfg.numAttrs = verbose ? 0 : 1;         // behind our own Z pass, which triggers its dependents early
-#define EDT_FIXUP(B, T)                                                                                          \
-    CUDA_TRY(cudaLaunchKernelEx(&fcfg, slab_fixup_kernel<B>, static_cast<const T*>(labels_dev), f_dev, plane, (int)sz, \
-                                halo, w2, has_lo, has_hi, set_lo, set_hi, L, step, flag_from_lo, flag_from_hi, kflags, \
-                                status_dev))
-    switch (label_bytes) {
-      case 1: EDT_FIXUP(1, uint8_t); break;
-      case 2: EDT_FIXUP(2, uint16_t); break;
-      case 4: EDT_FIXUP(4, uint32_t); break;
-      default: EDT_FIXUP(8, uint64_t); break;
-    }
-#undef EDT_FIXUP
+    cudaLaunchAttribute fattr;
+    fattr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    fattr.val.programmaticStreamSerializationAllowed = 1;
+    // PDL behind our own Z pass, which triggers its dependents early
+    const cudaLaunchConfig_t fcfg = {grid, dim3(256), 0, stream, &fattr, verbose ? 0u : 1u};
+    CUDA_TRY(with_label_width(label_bytes, [&](auto lw) {
+      using LW = decltype(lw);
+      return cudaLaunchKernelEx(&fcfg, slab_fixup_kernel<LW::Bytes>, static_cast<const typename LW::T*>(labels_dev),
+                                f_dev, plane, (int)sz, halo, w2, has_lo, has_hi, set_lo, set_hi, L, step, flag_from_lo,
+                                flag_from_hi, kflags, status_dev);
+    }));
     CUDA_TRY(cudaGetLastError());
     nvtx_pop();
   }
@@ -1296,20 +1273,12 @@ int edtb200_label_stats(const void* labels_dev, int label_bytes, const float* dt
   const int64_t total = sx * sy * sz;
   if (total > 0) {
     const unsigned blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)dc->sm_count * 16);
-    switch (label_bytes) {
-#define EDT_STATS(B, T)                                                                                       \
-      case B:                                                                                                 \
-        label_stats_kernel<B><<<blocks, 256, 0, stream>>>(static_cast<const T*>(labels_dev), dt_dev, total,   \
-                                                          (int)sx, (int)sy, t);                               \
-        label_argmax_kernel<B><<<blocks, 256, 0, stream>>>(static_cast<const T*>(labels_dev), dt_dev, total, t); \
-        break;
-      EDT_STATS(1, uint8_t) EDT_STATS(2, uint16_t) EDT_STATS(4, uint32_t)
-      default:
-        label_stats_kernel<8><<<blocks, 256, 0, stream>>>(static_cast<const uint64_t*>(labels_dev), dt_dev, total,
-                                                          (int)sx, (int)sy, t);
-        label_argmax_kernel<8><<<blocks, 256, 0, stream>>>(static_cast<const uint64_t*>(labels_dev), dt_dev, total, t);
-#undef EDT_STATS
-    }
+    with_label_width(label_bytes, [&](auto lw) {
+      using LW = decltype(lw);
+      const auto* lab = static_cast<const typename LW::T*>(labels_dev);
+      label_stats_kernel<LW::Bytes><<<blocks, 256, 0, stream>>>(lab, dt_dev, total, (int)sx, (int)sy, t);
+      label_argmax_kernel<LW::Bytes><<<blocks, 256, 0, stream>>>(lab, dt_dev, total, t);
+    });
   }
   label_table_finish_kernel<<<(capacity + 255) / 256, 256, 0, stream>>>(t);
   CUDA_TRY(cudaGetLastError());
@@ -1337,12 +1306,12 @@ int edtb200_label_extract(const void* labels_dev, int label_bytes, const float* 
   const int bx = b[3] - b[0] + 1, by = b[4] - b[1] + 1, bz = b[5] - b[2] + 1;
   const int64_t rows = (int64_t)by * bz;
   const unsigned blocks = (unsigned)std::min<int64_t>((rows + 7) / 8, (int64_t)dc->sm_count * 16);
-  switch (label_bytes) {
-    case 1: label_extract_kernel<1><<<blocks, 256, 0, stream>>>(static_cast<const uint8_t*>(labels_dev), dt_dev, out_dev, (int)sx, (int)sy, b[0], b[1], b[2], bx, by, bz, key, erase); break;
-    case 2: label_extract_kernel<2><<<blocks, 256, 0, stream>>>(static_cast<const uint16_t*>(labels_dev), dt_dev, out_dev, (int)sx, (int)sy, b[0], b[1], b[2], bx, by, bz, key, erase); break;
-    case 4: label_extract_kernel<4><<<blocks, 256, 0, stream>>>(static_cast<const uint32_t*>(labels_dev), dt_dev, out_dev, (int)sx, (int)sy, b[0], b[1], b[2], bx, by, bz, key, erase); break;
-    default: label_extract_kernel<8><<<blocks, 256, 0, stream>>>(static_cast<const uint64_t*>(labels_dev), dt_dev, out_dev, (int)sx, (int)sy, b[0], b[1], b[2], bx, by, bz, key, erase); break;
-  }
+  with_label_width(label_bytes, [&](auto lw) {
+    using LW = decltype(lw);
+    label_extract_kernel<LW::Bytes><<<blocks, 256, 0, stream>>>(static_cast<const typename LW::T*>(labels_dev), dt_dev,
+                                                                out_dev, (int)sx, (int)sy, b[0], b[1], b[2], bx, by,
+                                                                bz, key, erase);
+  });
   CUDA_TRY(cudaGetLastError());
   return 0;
 }

@@ -94,10 +94,5 @@ template <int Bytes>
 int launch_later(const void* labels, float* f, const LineGeom& g0, float w, int border_lo, int border_hi,
                  int flags, DeviceCache& dc, cudaStream_t stream, bool pdl, double fmax);
 
-// Shared memory of one tile of `tx` lines (see later_axis_tile_kernel); tile_path_ok tells whether
-// launch_later takes the shared-memory tile kernel for this geometry.
-size_t tile_smem_bytes(int n, int tx, int rows_alloc);
-bool tile_path_ok(const LineGeom& g, const DeviceCache& dc);
-
 }  // namespace host
 }  // namespace edtb200
