@@ -129,20 +129,41 @@ def nvl(val, default_val):
 # host-side logic mirrored from the reference's Cython layer
 # ---------------------------------------------------------------------------------------
 
-def _label_view(data):
+def _label_view(data, voxel_graph=False):
   """Labels as raw unsigned integers (src/edt.pyx:670-732): signed ints are reinterpreted,
   bool is one byte, floats are compared by value (so -0.0 is folded onto +0.0 first).
-  Returns None for dtypes the reference does not dispatch on (it then returns zeros)."""
+  With a voxel graph the labels only say foreground (> 0) or background
+  (src/edt_voxel_graph.hpp:76, 151), so floats are kept as they are and `_run` marks them
+  EDTB200_LABELS_FLOAT.  Returns None for dtypes the reference does not dispatch on (it then
+  returns zeros)."""
   dt = data.dtype
   if dt == np.bool_:
     return data.view(np.uint8)
   if dt.kind in "iu" and dt.itemsize in (1, 2, 4, 8):
     return data.view(np.dtype("u%d" % dt.itemsize))
-  if dt == np.float32:
-    return (data + np.float32(0)).view(np.uint32)
-  if dt == np.float64:
-    return (data + np.float64(0)).view(np.uint64)
+  if dt == np.float32 or dt == np.float64:
+    return data if voxel_graph else (data + dt.type(0)).view(np.dtype("u%d" % dt.itemsize))
   return None
+
+
+def _check_dims(dims, voxel_graph=None):
+  """The reference's dimension checks (src/edt.pyx:291-292, 310)."""
+  if voxel_graph is not None and dims not in (2, 3):
+    raise TypeError("Voxel connectivity graph is only supported for 2D and 3D. Got {}.".format(dims))
+  if dims < 1 or dims > 3:
+    raise TypeError("Multi-Label EDT library only supports up to 3 dimensions got {}.".format(dims))
+
+
+def _anisotropy(anisotropy, dims):
+  """Weights of an array of `dims` dimensions, in array axis order (src/edt.pyx:276-310): None
+  means ones, and a 1-D array takes a scalar or the first entry of a sequence.  Anything else is
+  passed on for _x_fastest to check (a scalar raises TypeError, a wrong length ValueError) once
+  the label dtype is known to be supported: for the others the reference returns zeros."""
+  if anisotropy is None:
+    return (1.0,) * dims
+  if dims == 1:
+    return (float(np.asarray(anisotropy).reshape(-1)[0]),)
+  return anisotropy
 
 
 def _x_fastest(shape, anisotropy, f_contiguous):
@@ -238,30 +259,31 @@ def _result_buffer(count):
   return np.frombuffer(block, dtype=np.float32, count=count)
 
 
-def _transform_host(data, anisotropy, black_border, flags, device):
-  nd = data.ndim
-  order = "F" if data.flags.f_contiguous else "C"
-  if not data.flags.c_contiguous and not data.flags.f_contiguous:
-    data = np.ascontiguousarray(data)
-  labels = _label_view(data)
-  if labels is None:
-    return np.zeros(data.shape, dtype=np.float32, order=order)
-  (sx, sy, sz), (wx, wy, wz) = _x_fastest(data.shape, anisotropy, order == "F")
-  out = _result_buffer(data.size)
-  lib = _lib()
-  if isinstance(device, (list, tuple, range)) or (isinstance(device, np.ndarray) and device.ndim == 1):
-    # several GPUs of this process share ONE host volume (edtb200_transform_multi): Z slabs for the
-    # X / Y passes, Y slabs for the Z pass, re-partitioned over NVLink; exact for any input
-    devs = [int(d) for d in device]
-    arr = (ctypes.c_int * len(devs))(*devs)
-    _check(lib.edtb200_transform_multi(
-      labels.ctypes.data, labels.dtype.itemsize, nd, sx, sy, sz, wx, wy, wz,
-      int(bool(black_border)), int(flags), out.ctypes.data, arr, len(devs)))
-    return out.reshape(data.shape, order=order)
-  _check(lib.edtb200_transform(
-    labels.ctypes.data, labels.dtype.itemsize, nd, sx, sy, sz, wx, wy, wz,
-    int(bool(black_border)), int(flags), out.ctypes.data, int(device), None))
-  return out.reshape(data.shape, order=order)
+def _run(labels, graph, dims, weights, black_border, flags, out, device=None):
+  """The one Python call site of edtb200_transform and, with a `graph`, of
+  edtb200_transform_voxel_graph.  `labels`, `graph` and `out` are numpy arrays, transformed on GPU
+  `device` before the call returns, or torch CUDA tensors, transformed asynchronously on their own
+  device and its current stream.  `dims` and `weights` are _x_fastest's."""
+  if isinstance(labels, np.ndarray):
+    def ptr(a):
+      return a.ctypes.data
+    stream, floating = None, labels.dtype.kind == "f"
+  else:
+    import torch
+
+    def ptr(a):
+      return a.data_ptr()
+    flags |= FLAG_LABELS_ON_DEVICE | FLAG_OUT_ON_DEVICE
+    device, floating = labels.device.index, labels.is_floating_point()
+    stream = ctypes.c_void_p(torch.cuda.current_stream(labels.device).cuda_stream)
+  if floating:                     # only with a graph: the labels are compared as floats (> 0)
+    flags |= FLAG_LABELS_FLOAT
+  (sx, sy, sz), (wx, wy, wz) = dims, weights
+  rest = (sx, sy, sz, wx, wy, wz, int(bool(black_border)), int(flags), ptr(out), int(device), stream)
+  if graph is None:
+    _check(_lib().edtb200_transform(ptr(labels), labels.itemsize, labels.ndim, *rest))
+  else:
+    _check(_lib().edtb200_transform_voxel_graph(ptr(labels), labels.itemsize, ptr(graph), labels.ndim, *rest))
 
 
 def _graph_bytes(voxel_graph, order):
@@ -271,30 +293,35 @@ def _graph_bytes(voxel_graph, order):
   return g.view(np.uint8) if g.dtype in (np.uint8, np.int8) else g.astype(np.uint8)
 
 
-def _transform_voxel_graph_host(data, voxel_graph, anisotropy, black_border, flags, device):
-  """__edt2dsq_voxel_graph / __edt3dsq_voxel_graph, src/edt.pyx:514-620, 736-844."""
+def _transform_host(data, voxel_graph, anisotropy, black_border, flags, device):
+  """A numpy array, answered in its memory order: Fortran order keeps the axes, anything else is
+  read in C order (src/edt.pyx:651-664), strided input after a copy.  With a voxel graph this is
+  __edt2dsq_voxel_graph / __edt3dsq_voxel_graph, src/edt.pyx:514-620, 736-844."""
   order = "F" if data.flags.f_contiguous else "C"
   if not data.flags.c_contiguous and not data.flags.f_contiguous:
     data = np.ascontiguousarray(data)
-  graph = _graph_bytes(voxel_graph, order)
-  if graph.shape != data.shape:
-    raise ValueError("voxel_graph must have the shape of data")
-  dt = data.dtype
-  if dt == np.bool_:
-    labels = data.view(np.uint8)
-  elif dt.kind in "iu" and dt.itemsize in (1, 2, 4, 8):
-    labels = data.view(np.dtype("u%d" % dt.itemsize))
-  elif dt in (np.float32, np.float64):
-    labels, flags = data, flags | FLAG_LABELS_FLOAT
+  graph = None
+  if voxel_graph is not None:
+    graph = _graph_bytes(voxel_graph, order)
+    if graph.shape != data.shape:
+      raise ValueError("voxel_graph must have the shape of data")
+  labels = _label_view(data, voxel_graph=graph is not None)
+  if labels is None:
+    return np.zeros(data.shape, dtype=np.float32, order=order)
+  dims, weights = _x_fastest(data.shape, anisotropy, order == "F")
+  out = _result_buffer(data.size) if graph is None else np.empty(data.size, dtype=np.float32)
+  if graph is None and (isinstance(device, (list, tuple, range))
+                        or (isinstance(device, np.ndarray) and device.ndim == 1)):
+    # several GPUs of this process share ONE host volume (edtb200_transform_multi): Z slabs for the
+    # X / Y passes, Y slabs for the Z pass, re-partitioned over NVLink; exact for any input
+    devs = [int(d) for d in device]
+    _check(_lib().edtb200_transform_multi(
+      labels.ctypes.data, labels.itemsize, data.ndim, *dims, *weights, int(bool(black_border)), int(flags),
+      out.ctypes.data, (ctypes.c_int * len(devs))(*devs), len(devs)))
   else:
-    return np.zeros(data.shape, dtype=np.float32, order=order)   # no branch in the reference either
-  (sx, sy, sz), (wx, wy, wz) = _x_fastest(data.shape, anisotropy, order == "F")
-  out = np.empty(data.size, dtype=np.float32)
-  if isinstance(device, (list, tuple)):
-    device = device[0]                      # the graph transform runs on one GPU
-  _check(_lib().edtb200_transform_voxel_graph(
-    labels.ctypes.data, labels.dtype.itemsize, graph.ctypes.data, data.ndim, sx, sy, sz, wx, wy, wz,
-    int(bool(black_border)), int(flags), out.ctypes.data, int(device), None))
+    if isinstance(device, (list, tuple)):
+      device = device[0]                      # the graph transform runs on one GPU
+    _run(labels, graph, dims, weights, black_border, flags, out, device)
   return out.reshape(data.shape, order=order)
 
 
@@ -324,97 +351,60 @@ def _device_array(data):
   return None
 
 
-def _front_door_device(t, anisotropy, black_border, voxel_graph, flags, fixed_dims):
-  """Device-resident input to the reference-named functions: same semantics, result returned as a
-  torch CUDA tensor (which itself exports DLPack and `__cuda_array_interface__`).  A Fortran-ordered
-  array is transformed through its transposed (C-ordered) view with the anisotropy reversed, which
-  is exactly the axis mapping of src/edt.pyx:651-664, so the memory order is preserved without a copy."""
+def _transform_device(t, voxel_graph, anisotropy, black_border, flags, device=None):
+  """A torch CUDA tensor, transformed on its own device (`device` is not used) and current stream,
+  answered as a torch CUDA tensor in its memory order (which itself exports DLPack and
+  `__cuda_array_interface__`).  As on the host, Fortran order keeps the axes and anything else is
+  read in C order (src/edt.pyx:651-664), so a Fortran-ordered tensor is not copied."""
   import torch
-  dims = t.dim()
-  if fixed_dims is not None and dims != fixed_dims:
-    raise ValueError("expected a %d-D array, got %d-D" % (fixed_dims, dims))
-  if dims > 3:
-    raise TypeError("Multi-Label EDT library only supports up to 3 dimensions got {}.".format(dims))
-  if voxel_graph is not None and dims not in (2, 3):
-    raise TypeError("Voxel connectivity graph is only supported for 2D and 3D. Got {}.".format(dims))
-  if t.numel() == 0:
-    return torch.zeros(t.shape, dtype=torch.float32, device=t.device)
-  if t.dtype in (torch.float32, torch.float64):
-    if voxel_graph is not None:
-      # with a graph the labels only say foreground / background, and for floats the reference
-      # tests `labels[loc] > 0` (src/edt_voxel_graph.hpp:76, 151): negative values and NaN are
-      # background, exactly as on the host path (EDTB200_LABELS_FLOAT)
-      t = (t > 0).to(torch.uint8)
-    else:
-      # labels compare by value (src/edt.pyx:704-722): fold -0.0 onto +0.0, then use the raw bits
-      t = (t + 0).view(torch.int32 if t.dtype == torch.float32 else torch.int64)
-  if anisotropy is None:
-    anisotropy = (1.0,) * dims
-  elif np.ndim(anisotropy) == 0:
-    anisotropy = (float(anisotropy),)
-  else:
-    anisotropy = tuple(float(a) for a in anisotropy)
-  if len(anisotropy) != dims:
-    raise ValueError("anisotropy must have one entry per dimension")
-  fortran = dims > 1 and not t.is_contiguous() and t.permute(*reversed(range(dims))).is_contiguous()
-  if fortran:
-    t = t.permute(*reversed(range(dims)))
-    anisotropy = tuple(reversed(anisotropy))
   graph = None
   if voxel_graph is not None:
     graph = _device_array(voxel_graph)
     if graph is None:
       graph = torch.as_tensor(np.ascontiguousarray(voxel_graph), device=t.device)
+    if graph.shape != t.shape or graph.device != t.device:
+      raise ValueError("voxel_graph must have the shape and device of data")
     if graph.dtype not in (torch.uint8, torch.int8):
       graph = graph.to(torch.uint8)
-    if fortran:
-      graph = graph.permute(*reversed(range(dims)))
-    graph = graph.contiguous()
-  sqrt, signed = bool(flags & FLAG_SQRT), bool(flags & FLAG_SIGNED)
-  if graph is not None and signed:       # f(data) - f(data == 0), src/edt.pyx:147-158
-    out = edt_cuda(t, anisotropy, black_border, sqrt=sqrt, voxel_graph=graph)
-    out -= edt_cuda(t == 0, anisotropy, black_border, sqrt=sqrt, voxel_graph=graph)
+  labels = _torch_label_view(t, voxel_graph=graph is not None)
+  if labels is None:
+    return torch.zeros(t.shape, dtype=torch.float32, device=t.device)
+  rev = tuple(reversed(range(labels.dim())))
+  fortran = labels.dim() > 1 and not labels.is_contiguous() and labels.permute(rev).is_contiguous()
+  if fortran:
+    graph = None if graph is None else graph.permute(rev).contiguous().permute(rev)
   else:
-    out = edt_cuda(t, anisotropy, black_border, sqrt=sqrt, signed=signed, voxel_graph=graph)
-  return out.permute(*reversed(range(dims))) if fortran else out
+    labels = labels.contiguous()
+    graph = None if graph is None else graph.contiguous()
+  dims, weights = _x_fastest(labels.shape, anisotropy, fortran)
+  out = torch.empty_like(labels, dtype=torch.float32)        # same strides as the labels
+  _run(labels, graph, dims, weights, black_border, flags, out)
+  return out
 
 
 def _front_door(data, anisotropy, black_border, voxel_graph, flags, device, fixed_dims=None):
-  """Argument handling of edtsq(), src/edt.pyx:276-310."""
+  """Argument handling of edtsq(), src/edt.pyx:276-310, for host arrays and device-resident input
+  alike; the result is a numpy array or a torch CUDA tensor, as the input is."""
   on_device = _device_array(data)
-  if on_device is not None:
-    return _front_door_device(on_device, anisotropy, black_border, voxel_graph, flags, fixed_dims)
-  if isinstance(data, list):
-    data = np.array(data)
-  data = np.asarray(data)
+  data = np.asarray(data) if on_device is None else on_device
   dims = data.ndim
   if fixed_dims is not None and dims != fixed_dims:
     raise ValueError("expected a %d-D array, got %d-D" % (fixed_dims, dims))
-  if data.size == 0:
-    return np.zeros(shape=data.shape, dtype=np.float32)
-  if voxel_graph is not None:
-    if dims not in (2, 3):
-      raise TypeError("Voxel connectivity graph is only supported for 2D and 3D. Got {}.".format(dims))
-    anisotropy = nvl(anisotropy, (1.0,) * dims)
-    if flags & FLAG_SIGNED:
-      # sdf / sdfsq with a graph: f(data) - f(data == 0), both under the graph (src/edt.pyx:147-158)
-      dt = _transform_voxel_graph_host(data, voxel_graph, anisotropy, black_border, flags & ~FLAG_SIGNED, device)
-      dt -= _transform_voxel_graph_host(data == 0, voxel_graph, anisotropy, black_border, flags & ~FLAG_SIGNED,
-                                        device)
-      return dt
-    return _transform_voxel_graph_host(data, voxel_graph, anisotropy, black_border, flags, device)
-  if dims == 1:
-    anisotropy = nvl(anisotropy, 1.0)
-    if np.ndim(anisotropy) != 0:
-      anisotropy = np.asarray(anisotropy).reshape(-1)[0]
-    anisotropy = (float(anisotropy),)
-  elif dims == 2:
-    anisotropy = nvl(anisotropy, (1.0, 1.0))
-  elif dims == 3:
-    anisotropy = nvl(anisotropy, (1.0, 1.0, 1.0))
-  else:
-    raise TypeError("Multi-Label EDT library only supports up to 3 dimensions got {}.".format(dims))
-  return _transform_host(data, anisotropy, black_border, flags, device)
+  if 0 in data.shape:
+    if on_device is None:
+      return np.zeros(shape=data.shape, dtype=np.float32)
+    import torch
+    return torch.zeros(data.shape, dtype=torch.float32, device=data.device)
+  _check_dims(dims, voxel_graph)
+  anisotropy = _anisotropy(anisotropy, dims)
+  transform = _transform_host if on_device is None else _transform_device
+  if voxel_graph is not None and flags & FLAG_SIGNED:
+    # sdf / sdfsq with a graph: f(data) - f(data == 0), both under the graph (src/edt.pyx:147-158)
+    flags &= ~FLAG_SIGNED
+    dt = transform(data, voxel_graph, anisotropy, black_border, flags, device)
+    dt -= transform(data == 0, voxel_graph, anisotropy, black_border, flags, device)
+    return dt
+  return transform(data, voxel_graph, anisotropy, black_border, flags, device)
 
 
 # ---------------------------------------------------------------------------------------
@@ -503,6 +493,18 @@ def _torch_label_bytes(torch):
   return _TORCH_LABEL_BYTES
 
 
+def _torch_label_view(t, voxel_graph=False):
+  """The torch counterpart of _label_view: `t` itself for integer and bool labels, whose raw bits
+  are the labels; floats compared by value (-0.0 folded onto +0.0) as their raw bits, or, with a
+  voxel graph, kept as they are; None for dtypes the reference does not dispatch on."""
+  import torch
+  if t.dtype in _torch_label_bytes(torch):
+    return t
+  if t.dtype == torch.float32 or t.dtype == torch.float64:
+    return t if voxel_graph else (t + 0).view(torch.int32 if t.dtype == torch.float32 else torch.int64)
+  return None
+
+
 def edt_cuda(labels, anisotropy=None, black_border=False, *, sqrt=False, signed=False, out=None,
              voxel_graph=None):
   """Transform a C-contiguous integer/bool torch CUDA tensor of 1-3 dims on its own device
@@ -514,12 +516,10 @@ def edt_cuda(labels, anisotropy=None, black_border=False, *, sqrt=False, signed=
   if not (isinstance(labels, torch.Tensor) and labels.is_cuda):
     raise TypeError("edt_cuda expects a torch CUDA tensor")
   nd = labels.dim()
-  if nd < 1 or nd > 3:
-    raise TypeError("Multi-Label EDT library only supports up to 3 dimensions got {}.".format(nd))
+  _check_dims(nd)
   if not labels.is_contiguous():
     labels = labels.contiguous()
-  nbytes = _torch_label_bytes(torch).get(labels.dtype)
-  if nbytes is None:
+  if labels.dtype not in _torch_label_bytes(torch):
     raise TypeError("edt_cuda: unsupported label dtype %s" % labels.dtype)
   if out is None:
     out = torch.empty(labels.shape, dtype=torch.float32, device=labels.device)
@@ -528,33 +528,17 @@ def edt_cuda(labels, anisotropy=None, black_border=False, *, sqrt=False, signed=
     raise ValueError("edt_cuda: `out` must be a contiguous float32 CUDA tensor of the same shape/device")
   if labels.numel() == 0:
     return out
-  if anisotropy is None:
-    anisotropy = (1.0,) * nd
-  elif nd == 1 and np.ndim(anisotropy) == 0:
-    anisotropy = (float(anisotropy),)
-  (sx, sy, sz), (wx, wy, wz) = _x_fastest(labels.shape, anisotropy, False)
-  flags = FLAG_LABELS_ON_DEVICE | FLAG_OUT_ON_DEVICE
-  if sqrt:
-    flags |= FLAG_SQRT
-  if signed:
-    flags |= FLAG_SIGNED
-  stream = torch.cuda.current_stream(labels.device).cuda_stream
+  dims, weights = _x_fastest(labels.shape, _anisotropy(anisotropy, nd), False)
+  flags = (FLAG_SQRT if sqrt else 0) | (FLAG_SIGNED if signed else 0)
   if voxel_graph is not None:
-    if nd not in (2, 3):
-      raise TypeError("Voxel connectivity graph is only supported for 2D and 3D. Got {}.".format(nd))
+    _check_dims(nd, voxel_graph)
     if signed:
       raise ValueError("edt_cuda: with voxel_graph, form f(labels) - f(labels == 0) from two calls")
     if not (isinstance(voxel_graph, torch.Tensor) and voxel_graph.device == labels.device
             and voxel_graph.dtype in (torch.uint8, torch.int8) and voxel_graph.shape == labels.shape):
       raise ValueError("edt_cuda: voxel_graph must be a uint8/int8 CUDA tensor shaped like labels")
     voxel_graph = voxel_graph.contiguous()
-    _check(_lib().edtb200_transform_voxel_graph(
-      labels.data_ptr(), nbytes, voxel_graph.data_ptr(), nd, sx, sy, sz, wx, wy, wz,
-      int(bool(black_border)), flags, out.data_ptr(), labels.device.index, ctypes.c_void_p(stream)))
-    return out
-  _check(_lib().edtb200_transform(
-    labels.data_ptr(), nbytes, nd, sx, sy, sz, wx, wy, wz, int(bool(black_border)), flags,
-    out.data_ptr(), labels.device.index, ctypes.c_void_p(stream)))
+  _run(labels, voxel_graph, dims, weights, black_border, flags, out)
   return out
 
 
@@ -570,8 +554,7 @@ def transform_batch(volumes, anisotropy=None, black_border=False, *, sqrt=False,
   if not vols:
     return []
   first = vols[0]
-  if first.ndim < 1 or first.ndim > 3:
-    raise TypeError("Multi-Label EDT library only supports up to 3 dimensions got {}.".format(first.ndim))
+  _check_dims(first.ndim)
   order = "F" if first.flags.f_contiguous else "C"
   fixed = []
   for v in vols:
@@ -603,11 +586,7 @@ def transform_batch(volumes, anisotropy=None, black_border=False, *, sqrt=False,
       o[...] = 0
     return outs
   nd = first.ndim
-  if anisotropy is None:
-    anisotropy = (1.0,) * nd
-  elif nd == 1 and np.ndim(anisotropy) == 0:
-    anisotropy = (float(anisotropy),)
-  (sx, sy, sz), (wx, wy, wz) = _x_fastest(first.shape, anisotropy, order == "F")
+  (sx, sy, sz), (wx, wy, wz) = _x_fastest(first.shape, _anisotropy(anisotropy, nd), order == "F")
   n = len(views)
   lab_ptrs = (ctypes.c_void_p * n)(*[v.ctypes.data for v in views])
   out_ptrs = (ctypes.c_void_p * n)(*[o.ctypes.data for o in outs])
@@ -641,7 +620,7 @@ def label_stats_cuda(labels, dt):
   labels = labels.contiguous()
   dt = dt.contiguous().to(torch.float32)
   nd = labels.dim()
-  dims = [int(d) for d in labels.shape][::-1] + [1] * (3 - nd)          # sx, sy, sz
+  (sx, sy, sz), _ = _x_fastest(labels.shape, (1.0,) * nd, False)
   dev = labels.device
   stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
   capacity = 1024
@@ -652,9 +631,9 @@ def label_stats_cuda(labels, dt):
     argmax = torch.empty(capacity, dtype=torch.int64, device=dev)
     box = torch.empty((capacity, 6), dtype=torch.int32, device=dev)
     overflow = torch.zeros(1, dtype=torch.int32, device=dev)
-    _check(_lib().edtb200_label_stats(labels.data_ptr(), nbytes, dt.data_ptr(), dims[0], dims[1], dims[2],
-                                      capacity, keys.data_ptr(), count.data_ptr(), mx.data_ptr(),
-                                      argmax.data_ptr(), box.data_ptr(), overflow.data_ptr(), dev.index, stream))
+    _check(_lib().edtb200_label_stats(labels.data_ptr(), nbytes, dt.data_ptr(), sx, sy, sz, capacity,
+                                      keys.data_ptr(), count.data_ptr(), mx.data_ptr(), argmax.data_ptr(),
+                                      box.data_ptr(), overflow.data_ptr(), dev.index, stream))
     used = int((keys != 0).sum().item())
     if int(overflow.item()) == 0 and 2 * used <= capacity:
       break
@@ -675,17 +654,10 @@ def _unsigned_sort_key(torch, keys, nbytes):
   return keys ^ torch.tensor(-0x8000000000000000, dtype=torch.int64, device=keys.device)
 
 
-def _label_scalar(torch, key, dtype):
-  """The label value a table key (the label's raw bits, zero-extended) stands for."""
-  nbytes = torch.empty((), dtype=dtype).element_size()
-  raw = np.array([key & ((1 << (8 * nbytes)) - 1)], dtype=np.dtype("u%d" % nbytes))
-  if dtype == torch.bool:
-    return bool(raw[0])
-  if dtype.is_floating_point:
-    return float(raw.view(np.dtype("f%d" % nbytes))[0])
-  if dtype == torch.uint8:
-    return int(raw[0])
-  return int(raw.view(np.dtype("i%d" % nbytes))[0])      # torch's other integer types are signed
+def _label_scalar(key, dtype):
+  """The label of numpy `dtype` that a table key (the label's raw bits, zero-extended) stands for."""
+  raw = np.array([key & ((1 << (8 * dtype.itemsize)) - 1)], dtype=np.dtype("u%d" % dtype.itemsize))
+  return raw.view(dtype)[0]
 
 
 def each_cuda(labels, dt, in_place=False, *, _stats=None):
@@ -701,8 +673,11 @@ def each_cuda(labels, dt, in_place=False, *, _stats=None):
   labels = labels.contiguous()
   dt = dt.contiguous().to(torch.float32)
   nbytes = _torch_label_bytes(torch)[labels.dtype]
+  # labels are reported as Python values: bool, uint8 unsigned, torch's other integer types signed
+  value_type = np.dtype(bool if labels.dtype == torch.bool else "u1" if labels.dtype == torch.uint8 else
+                        "i%d" % nbytes)
   nd = labels.dim()
-  dims = [int(d) for d in labels.shape][::-1] + [1] * (3 - nd)
+  (sx, sy, sz), _ = _x_fastest(labels.shape, (1.0,) * nd, False)
   dev = labels.device
   keys = stats["labels"].tolist()
   boxes = stats["box"].tolist()
@@ -721,13 +696,13 @@ def each_cuda(labels, dt, in_place=False, *, _stats=None):
         cbox = (ctypes.c_int * 6)(*(lo + hi))
         out = img if in_place else torch.zeros(labels.shape, dtype=torch.float32, device=dev)
         if in_place and prev is not None:
-          _check(lib.edtb200_label_extract(labels.data_ptr(), nbytes, dt.data_ptr(), dims[0], dims[1], dims[2],
+          _check(lib.edtb200_label_extract(labels.data_ptr(), nbytes, dt.data_ptr(), sx, sy, sz,
                                            ctypes.c_uint64(0), prev, 1, out.data_ptr(), dev.index, stream))
-        _check(lib.edtb200_label_extract(labels.data_ptr(), nbytes, dt.data_ptr(), dims[0], dims[1], dims[2],
+        _check(lib.edtb200_label_extract(labels.data_ptr(), nbytes, dt.data_ptr(), sx, sy, sz,
                                          ctypes.c_uint64(key & 0xffffffffffffffff), cbox, 0, out.data_ptr(),
                                          dev.index, stream))
         prev = cbox
-        yield (_label_scalar(torch, key, labels.dtype), out)
+        yield (_label_scalar(key, value_type).item(), out)
 
   return DeviceImageIterator()
 
@@ -750,8 +725,7 @@ def each(labels, dt, in_place=False, *, device=0):
   dt = np.asarray(dt)
   if labels.shape != dt.shape:
     raise ValueError("labels and dt must have the same shape")
-  if labels.ndim < 1 or labels.ndim > 3:
-    raise TypeError("Multi-Label EDT library only supports up to 3 dimensions got {}.".format(labels.ndim))
+  _check_dims(labels.ndim)
   order = "F" if labels.flags.f_contiguous else "C"
   view = _label_view(labels)
   if view is None or torch is None:
@@ -760,20 +734,13 @@ def each(labels, dt, in_place=False, *, device=0):
   mem = view.T if order == "F" else view
   dmem = dt.T if order == "F" else dt
   dev = torch.device("cuda", int(device))
-  signed = {1: torch.uint8, 2: torch.int16, 4: torch.int32, 8: torch.int64}[view.dtype.itemsize]
-  raw = np.ascontiguousarray(mem)
-  lab_t = torch.from_numpy(raw.view(np.dtype("i%d" % raw.dtype.itemsize) if raw.dtype.itemsize > 1 else np.uint8)).to(dev)
-  assert lab_t.dtype == signed
+  lab_t = torch.from_numpy(np.ascontiguousarray(mem)).to(dev)
   dt_t = torch.from_numpy(np.ascontiguousarray(dmem, dtype=np.float32)).to(dev)
   stats = label_stats_cuda(lab_t, dt_t)
   keys = stats["labels"].tolist()
   boxes = stats["box"].tolist()
   nd = labels.ndim
   inner = each_cuda(lab_t, dt_t, in_place=True, _stats=stats)
-
-  def key_value(key):
-    # the device iterator reports the label's raw bits as an integer: back to the array's own dtype
-    return np.array([key & ((1 << (8 * view.dtype.itemsize)) - 1)], dtype=view.dtype).view(labels.dtype)[0]
 
   class ImageIterator:
     def __len__(self):
@@ -793,11 +760,11 @@ def each(labels, dt, in_place=False, *, device=0):
           img[host_sl] = host_sub
           img.setflags(write=0)
           prev = host_sl
-          yield (key_value(int(key)), img)
+          yield (_label_scalar(key, labels.dtype), img)
         else:
           out = np.zeros(labels.shape, dtype=np.float32, order=order)
           out[host_sl] = host_sub
-          yield (key_value(int(key)), out)
+          yield (_label_scalar(key, labels.dtype), out)
 
   return ImageIterator()
 

@@ -40,7 +40,7 @@ import ctypes
 import torch
 import torch.distributed as dist
 
-from . import FLAG_SIGNED, FLAG_SQRT, EDTError, _lib, _torch_label_bytes
+from . import FLAG_SIGNED, FLAG_SQRT, EDTError, _check, _lib, _torch_label_bytes
 
 
 def split_extent(total, parts):
@@ -64,41 +64,40 @@ class CudaPasses:
   def _stream(self):
     return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-  def _check(self, rc):
-    if rc != 0:
-      raise EDTError(self.lib.edtb200_last_error().decode("utf-8", "replace"))
+  @staticmethod
+  def _labels(labels):
+    """Pointer, label width and (sx, sy, sz) of a C-contiguous (z, y, x) label tensor."""
+    sz, sy, sx = labels.shape
+    return labels.data_ptr(), _torch_label_bytes(torch)[labels.dtype], sx, sy, sz
 
   def empty_f32(self, shape):
     return torch.empty(shape, dtype=torch.float32, device=self.device)
 
   def pass_first(self, labels, f, wx, black_border, signed):
-    sz, sy, sx = labels.shape
-    nbytes = _torch_label_bytes(torch)[labels.dtype]
-    self._check(self.lib.edtb200_pass_first(labels.data_ptr(), nbytes, sx, sy, sz, float(wx),
-                                            int(bool(black_border)), FLAG_SIGNED if signed else 0,
-                                            f.data_ptr(), self.device.index, self._stream()))
+    lab, nbytes, sx, sy, sz = self._labels(labels)
+    _check(self.lib.edtb200_pass_first(lab, nbytes, sx, sy, sz, float(wx),
+                                       int(bool(black_border)), FLAG_SIGNED if signed else 0,
+                                       f.data_ptr(), self.device.index, self._stream()))
 
   def pass_later(self, labels, f, axis, w, border_lo, border_hi, sqrt=False, negate=False):
-    sz, sy, sx = labels.shape
-    nbytes = _torch_label_bytes(torch)[labels.dtype]
+    lab, nbytes, sx, sy, sz = self._labels(labels)
     flags = (FLAG_SQRT if sqrt else 0) | (FLAG_SIGNED if negate else 0)
-    self._check(self.lib.edtb200_pass_later(labels.data_ptr(), nbytes, int(axis), sx, sy, sz, float(w),
-                                            int(bool(border_lo)), int(bool(border_hi)), flags,
-                                            f.data_ptr(), self.device.index, self._stream()))
+    _check(self.lib.edtb200_pass_later(lab, nbytes, int(axis), sx, sy, sz, float(w),
+                                       int(bool(border_lo)), int(bool(border_hi)), flags,
+                                       f.data_ptr(), self.device.index, self._stream()))
 
 
   def slab_step(self, labels, f, w_xyz, black_border, has_lo, has_hi, sqrt, signed, halo, sym_self, sym_lo, sym_hi,
                 step, status):
     """One fused slab step (edtb200_slab_step): X, Y, stage faces, Z, fix-up, on the current stream."""
-    sz, sy, sx = labels.shape
-    nbytes = _torch_label_bytes(torch)[labels.dtype]
+    lab, nbytes, sx, sy, sz = self._labels(labels)
     flags = (FLAG_SQRT if sqrt else 0) | (FLAG_SIGNED if signed else 0)
-    self._check(self.lib.edtb200_slab_step(labels.data_ptr(), nbytes, sx, sy, sz, float(w_xyz[0]), float(w_xyz[1]),
-                                           float(w_xyz[2]), int(bool(black_border)), int(bool(has_lo)),
-                                           int(bool(has_hi)), flags, f.data_ptr(), int(halo),
-                                           ctypes.c_void_p(sym_self), ctypes.c_void_p(sym_lo or None),
-                                           ctypes.c_void_p(sym_hi or None), ctypes.c_uint64(step),
-                                           status.data_ptr(), self.device.index, self._stream()))
+    _check(self.lib.edtb200_slab_step(lab, nbytes, sx, sy, sz, float(w_xyz[0]), float(w_xyz[1]),
+                                      float(w_xyz[2]), int(bool(black_border)), int(bool(has_lo)),
+                                      int(bool(has_hi)), flags, f.data_ptr(), int(halo),
+                                      ctypes.c_void_p(sym_self), ctypes.c_void_p(sym_lo or None),
+                                      ctypes.c_void_p(sym_hi or None), ctypes.c_uint64(step),
+                                      status.data_ptr(), self.device.index, self._stream()))
 
   def repartition(self, src, dst, ysplit, unpack=False):
     """Z slab (zc, sy, row) <-> the exchange layout of the transposition fallback, ONE launch
@@ -108,29 +107,27 @@ class CudaPasses:
     zc, sy = slab.shape[0], slab.shape[1]
     row_bytes = slab.shape[2] * slab.element_size()
     starts = (ctypes.c_int64 * (len(ysplit) + 1))(*([s for s, _ in ysplit] + [sy]))
-    self._check(self.lib.edtb200_slab_pack(src.data_ptr(), dst.data_ptr(), zc, sy, row_bytes, len(ysplit), starts,
-                                           1 if unpack else 0, self.device.index, self._stream()))
+    _check(self.lib.edtb200_slab_pack(src.data_ptr(), dst.data_ptr(), zc, sy, row_bytes, len(ysplit), starts,
+                                      1 if unpack else 0, self.device.index, self._stream()))
 
   def face_runs(self, labels, high_face, halo, signed, overflow, out=None):
     """uint8 (sy, sx) run lengths at one face; raises the device int `overflow` when too long."""
-    sz, sy, sx = labels.shape
-    nbytes = _torch_label_bytes(torch)[labels.dtype]
+    lab, nbytes, sx, sy, sz = self._labels(labels)
     m = out if out is not None else torch.empty((sy, sx), dtype=torch.uint8, device=self.device)
-    self._check(self.lib.edtb200_slab_face_runs(labels.data_ptr(), nbytes, sx, sy, sz, int(high_face), int(halo),
-                                                FLAG_SIGNED if signed else 0, m.data_ptr(),
-                                                overflow.data_ptr(), self.device.index, self._stream()))
+    _check(self.lib.edtb200_slab_face_runs(lab, nbytes, sx, sy, sz, int(high_face), int(halo),
+                                           FLAG_SIGNED if signed else 0, m.data_ptr(),
+                                           overflow.data_ptr(), self.device.index, self._stream()))
     return m
 
   def face_fixup(self, labels, f, high_face, halo, wz, sqrt, signed, nb_label, nb_m, nb_f, inexact):
     """`inexact` (device int32[1]) is raised when a run continues behind the halo AND the distances
     at the face are larger than the halo reaches, i.e. an unseen site could still win."""
-    sz, sy, sx = labels.shape
-    nbytes = _torch_label_bytes(torch)[labels.dtype]
+    lab, nbytes, sx, sy, sz = self._labels(labels)
     flags = (FLAG_SQRT if sqrt else 0) | (FLAG_SIGNED if signed else 0)
-    self._check(self.lib.edtb200_slab_face_fixup(labels.data_ptr(), nbytes, sx, sy, sz, int(high_face),
-                                                 int(halo), float(wz), flags, nb_label.data_ptr(),
-                                                 nb_m.data_ptr(), nb_f.data_ptr(), f.data_ptr(),
-                                                 inexact.data_ptr(), self.device.index, self._stream()))
+    _check(self.lib.edtb200_slab_face_fixup(lab, nbytes, sx, sy, sz, int(high_face),
+                                            int(halo), float(wz), flags, nb_label.data_ptr(),
+                                            nb_m.data_ptr(), nb_f.data_ptr(), f.data_ptr(),
+                                            inexact.data_ptr(), self.device.index, self._stream()))
 
 
 def _all_to_all(send_chunks, recv_chunks, group, peers=None):
